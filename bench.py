@@ -58,7 +58,15 @@ def parse():
     ap.add_argument("--ext-compare", action="store_true",
                     help="time the reference's own extensions rebuilt for sm_100a (oracle/_ref) against ours: SG shade, "
                          "raydirs, MVP raymarch (BASELINE config 4 shape); prints its own JSON line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (rendered images and the "
+                         "gradients the step returns) as DIR/<name>.npy, at most 64 MB in all, for every --config of "
+                         "--impl ours; one process only (--gpus 1): with more, each rank holds only its own views")
+    a = ap.parse_args()
+    if a.dump_outputs and (a.decoder or a.decoder_library or a.ext_compare or a.impl != "ours"):
+        ap.error("--dump-outputs applies to the timed path of --impl ours (not --decoder / --decoder-library / "
+                 "--ext-compare)")
+    return a
 
 
 FIELDS = (("primpos", 3), ("primqvec", 4), ("primscale", 3), ("opacity", 1), ("diff_color", 3), ("lobe_dirs", 3),
@@ -480,6 +488,39 @@ class OlatWorkload:
         return [rgb, alpha, depth], grad
 
 
+DUMP_BYTES = 64_000_000
+
+
+def _dump_one_process(args, world):
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of one process (each rank holds only its own views): "
+                         "run it with --gpus 1")
+
+
+def dump_outputs(out_dir, arrays):
+    """Write the named tensors a caller of the timed step receives as out_dir/<name>.npy (float32).  When they exceed
+    DUMP_BYTES, each is replaced by a fixed, seeded sample of its flattened elements (<name>.npy), gathered on the device,
+    and the sampled flat indices (<name>_index.npy), the budget shared in proportion to the sizes."""
+    total = sum(t.numel() for t in arrays.values())
+    budget = DUMP_BYTES - 2 * 128 * len(arrays)  # .npy headers
+    keep = 1.0 if total * 4 <= budget else budget / (total * 12.0)  # 4 B value + 8 B index per sampled element
+    os.makedirs(out_dir, exist_ok=True)
+    for k, t in arrays.items():
+        t = t.detach()
+        if keep < 1.0:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), int(t.numel() * keep), replace=False))
+            np.save(os.path.join(out_dir, k + "_index.npy"), idx.astype(np.int64))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, k + ".npy"), t.float().cpu().numpy())
+
+
+def head_outputs(imgs, grad):
+    """The images and the per-field gradient (dL/d decoded Gaussians) one step of run_ours returns, by name."""
+    arrays = dict(zip(("rgb", "alpha", "depth"), imgs))
+    arrays.update(("grad_" + k, v) for k, v in unpack(grad, grad.numel() // NCOL).items())
+    return arrays
+
+
 def _timeit_events(fn, reps, flush=None):
     ts = []
     for _ in range(reps):
@@ -515,6 +556,7 @@ def run_ours(args):
     from goliath_b200.dist import FrameExchange
 
     lib = _lib.lib()
+    _dump_one_process(args, world)
     wl = (OlatWorkload if args.config == "olat" else HeadWorkload)(args, rank, world, dev)
     G = wl.G
     steps = args.steps if args.steps is not None else (200 if wl.key == "head" else 10)
@@ -575,10 +617,12 @@ def run_ours(args):
         """per-step event pairs; e2e: the table comes from pinned host memory and the images go back, serially."""
         def one():
             static_in.copy_(host_packed if e2e else resident, non_blocking=True)
-            imgs, _ = run_step()
+            imgs, grad = run_step()
             if e2e:
                 for dst, src_t in zip(host_out, imgs):
                     dst.copy_(src_t, non_blocking=True)
+            return imgs, grad
+        last = None
         for _ in range(n_warm):
             one()
         torch.cuda.synchronize()
@@ -589,12 +633,12 @@ def run_ours(args):
             flush()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            one()
+            last = one()
             b.record()
             evs.append((a, b))
         torch.cuda.synchronize()
         per_step = [a.elapsed_time(b) for a, b in evs]
-        return sum(per_step), per_step, time.perf_counter() - t0
+        return sum(per_step), per_step, time.perf_counter() - t0, last
 
     # ---------------------------------------------------------------- N > 1: the exchange steps (goliath_b200.dist)
     def timed_exchange(e2e, n_steps, n_warm):
@@ -750,7 +794,10 @@ def run_ours(args):
     e2e_steps = max(min(steps, 20), steps // 4)
     collectives = None
     if world == 1:
-        ms_total, per_step, wall = timed_single(False, steps, warmup)
+        ms_total, per_step, wall, last = timed_single(False, steps, warmup)
+        if args.dump_outputs:  # before the later phases reuse the graph's output buffers
+            dump_outputs(args.dump_outputs, head_outputs(*last))
+        del last
         ms_e2e_serial = timed_single(True, e2e_steps, 3)[0] * steps / e2e_steps
         ms_e2e = timed_e2e_streamed_single(steps, warmup)
         h2d_rank = host_packed.numel() * 4
@@ -978,7 +1025,11 @@ def run_hand_mvp(args):
     with torch.no_grad():  # random-init weights; output biases set so the volume is semi-transparent and coloured
         adec.texbranch[-1].bias.fill_(float(args.mvp_density))
         rdec.texbranch[-1].bias.fill_(2.0)
-    params = [p for m in (penc, tdec, adec, rdec) for p in m.parameters()]
+    named = [("%s.%s" % (mn, pn), p) for mn, m in (("penc", penc), ("tdec", tdec), ("adec", adec), ("rdec", rdec))
+             for pn, p in m.named_parameters()]
+    params = [p for _, p in named]
+    _dump_one_process(args, world)
+    kept = {}
     gen = torch.Generator().manual_seed(54)
     host_pose = torch.randn(NCAM, 60, generator=gen)[sel].contiguous().pin_memory()
     host_cond = torch.rand(NCAM, 2, 64, 64, generator=gen)[sel].contiguous().pin_memory()  # view_cos_uv, ambient occlusion
@@ -996,7 +1047,7 @@ def run_hand_mvp(args):
         out = mvr.mvpraymarch(raypos, raydir, step_sz, tminmax, (primpos, primrot, primscale), tpl, None)
         return out, (raypos, raydir, tminmax, primpos, primrot, primscale, tpl)
 
-    def step(e2e):
+    def step(e2e, keep=False):
         if e2e:
             pose_d.copy_(host_pose, non_blocking=True)
             cond_d.copy_(host_cond, non_blocking=True)
@@ -1007,6 +1058,8 @@ def run_hand_mvp(args):
             dist.all_reduce(flat)
         if e2e:
             host_img.copy_(out.detach(), non_blocking=True)
+        if keep:  # --dump-outputs: the last timed step's rendered rgba and parameter gradients
+            kept.update({"rgba": out.detach()}, **{"grad_" + n: p.grad for n, p in named if p.grad is not None})
         for p in params:
             p.grad = None
 
@@ -1018,9 +1071,9 @@ def run_hand_mvp(args):
             dist.barrier()
         lib.gb_launch_count_reset()
         evs = []
-        for _ in range(n):
+        for i in range(n):
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record(); step(e2e); b.record()
+            a.record(); step(e2e, keep=bool(args.dump_outputs) and not e2e and i == n - 1); b.record()
             evs.append((a, b))
         torch.cuda.synchronize()
         launches = int(lib.gb_launch_count())
@@ -1035,6 +1088,9 @@ def run_hand_mvp(args):
     if rank == 0:
         proc, path = sample_clocks_start(local)
     ms_total, launches = timed(False, steps, warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: torch.cat(v) if isinstance(v, list) else v for k, v in kept.items()})
+        kept.clear()
     ms_e2e, _ = timed(True, steps, 3)
     clocks = sample_clocks_stop(proc, path) if rank == 0 else None
     ext = roof = None
@@ -1109,8 +1165,11 @@ def run_mvp_full(args):
     tpl.requires_grad_()
     step_sz = 1.0 / 2000.0
     host_img = torch.empty(max(V, 1), H, W, 4).pin_memory()
+    _dump_one_process(args, world)
+    kept = {}
 
-    def step(e2e):
+    def step(e2e, keep=False):
+        outs = []
         if e2e:
             if rank == 0:
                 tpl.data.copy_(host_tpl, non_blocking=True)   # the frame owner's decoded template arrives from the host
@@ -1123,6 +1182,8 @@ def run_mvp_full(args):
             out.backward(_ones_like(out))
             if e2e:
                 host_img[i].copy_(out.detach()[0], non_blocking=True)
+            if keep:
+                outs.append(out.detach())
         if world > 1:
             for t in (tpl, primpos, primrot, primscale):
                 if t.grad is None:
@@ -1130,6 +1191,9 @@ def run_mvp_full(args):
             dist.all_reduce(tpl.grad)
             small = torch.cat([primpos.grad.reshape(-1), primrot.grad.reshape(-1), primscale.grad.reshape(-1)])
             dist.all_reduce(small)
+        if keep:  # --dump-outputs: the last timed step's rendered rgba of every camera and the accumulated gradients
+            kept.update(rgba=outs, grad_template=tpl.grad, grad_primpos=primpos.grad, grad_primrot=primrot.grad,
+                        grad_primscale=primscale.grad)
         for t in (tpl, primpos, primrot, primscale):
             t.grad = None
 
@@ -1141,9 +1205,9 @@ def run_mvp_full(args):
             dist.barrier()
         lib.gb_launch_count_reset()
         evs = []
-        for _ in range(n):
+        for i in range(n):
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record(); step(e2e); b.record()
+            a.record(); step(e2e, keep=bool(args.dump_outputs) and not e2e and i == n - 1); b.record()
             evs.append((a, b))
         torch.cuda.synchronize()
         launches = int(lib.gb_launch_count())
@@ -1158,6 +1222,9 @@ def run_mvp_full(args):
     if rank == 0:
         proc, path = sample_clocks_start(local)
     ms_total, launches = timed(False, steps, warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: torch.cat(v) if isinstance(v, list) else v for k, v in kept.items()})
+        kept.clear()
     ms_e2e, _ = timed(True, steps, 3)
     clocks = sample_clocks_stop(proc, path) if rank == 0 else None
     ext = roof = None

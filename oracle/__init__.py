@@ -7,11 +7,13 @@ numpy-in / numpy-out wrappers over ``liboracle.so`` (plain C, built by ``oracle/
 ``-ffp-contract=off``).  Each C function cites the reference file:line it restates.
 
 Parity status per path (also in DESIGN.md):
-  * SG shade (sg_oracle.c)        — pinned on the GPU box against the reference kernels rebuilt into oracle/_ref
-  * splat path (splat_oracle.c)   — PARITY UNPINNED: gsplat==0.1.11 is a third-party dependency absent from
-                                    /root/reference; restated from its published algorithm (SURVEY.md App. A)
-  * raydirs / raymarch            — pinned against oracle/_ref (reference kernels) on the GPU box and against the
-                                    reference's inline PyTorch raymarcher fixtures (tests/golden)
+  * SG shade (sg_oracle.c)        — pinned on the GPU against recorded outputs of the reference kernels rebuilt
+                                    into oracle/_ref (tests/golden/ref_kernels_sg.npz)
+  * splat path (splat_oracle.c)   — PARITY UNPINNED: gsplat==0.1.11 is a third-party dependency absent from the
+                                    reference checkout; restated from its published algorithm (SURVEY.md App. A)
+  * raydirs / raymarch            — pinned on the GPU against recorded outputs of the reference kernels
+                                    (tests/golden/ref_kernels_{mvp,raymarch}.npz) and against the reference's inline
+                                    PyTorch raymarcher fixtures (tests/golden)
 """
 import ctypes
 import os

@@ -1,28 +1,35 @@
-"""Build the REFERENCE's own CUDA extensions for sm_100a into oracle/_ref/ (git-ignored, shipped to the GPU box).
+"""Build the REFERENCE's own CUDA extensions for sm_100a into oracle/_ref/ (git-ignored).
 
-TEST INFRASTRUCTURE ONLY.  Compiles the sources WHERE THEY LIE under /root/reference/extensions (nothing is copied
-into the repo) with the reference's own flags (setup.py of each extension: -use_fast_math where it says so,
--std=c++17, -lineinfo) except the gencode, which is sm_100a.  The outputs are the reference's pybind modules
-`sgutilslib`, `utilslib`, `mvpraymarchlib`; tests load them from oracle/_ref as the GPU witness that pins the
-oracle and the product kernels (tests/test_ref_witness_gpu.py) and bench.py times them as the reference arm of
-the extension-level ratios.  gsplat is third-party and absent: it cannot be built here.
+TEST INFRASTRUCTURE ONLY.  Compiles the sources WHERE THEY LIE under <reference>/extensions, a checkout of
+facebookresearch/goliath at $GOLIATH_REFERENCE or, by default, at the `reference_path` BASELINE.json records (nothing
+is copied into the repo), with the reference's own flags (setup.py of each
+extension: -use_fast_math where it says so, -std=c++17, -lineinfo) except the gencode, which is sm_100a.  The outputs
+are the reference's pybind modules `sgutilslib`, `utilslib`, `mvpraymarchlib`; tests/golden/make_ref_kernels_golden.py
+records their outputs as the fixtures the GPU tests compare our kernels against, and bench.py --ext-compare times them
+as the reference arm of the extension-level ratios.  gsplat is third-party and absent: it cannot be built here.
 
-It also byte-compiles the reference's L1 PYTHON wrappers (extensions/*/X.py and ca_code/utils/render_gsplat.py: the
-`autograd.Function`s that call into the pybind modules) to sourceless .pyc files under oracle/_ref/pyc/ — compiled
-artefacts like the .so files, no source text enters the repo — so that tests/test_dropins.py can run the reference's
-OWN wrappers, unchanged, over `goliath_b200.install_dropins()` on the GPU box (where /root/reference does not exist).
-
-Usage: python oracle/build_ref.py [sgutilslib utilslib mvpraymarchlib]
+Usage: [GOLIATH_REFERENCE=<goliath checkout>] python oracle/build_ref.py [sgutilslib utilslib mvpraymarchlib]
 """
+import json
 import os
 import subprocess
 import sys
 import sysconfig
 from concurrent.futures import ThreadPoolExecutor
 
-REF = "/root/reference/extensions"
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.path.join(HERE, "_ref")
+
+
+def reference_dir():
+    """$GOLIATH_REFERENCE, else the reference checkout BASELINE.json records."""
+    if os.environ.get("GOLIATH_REFERENCE"):
+        return os.environ["GOLIATH_REFERENCE"]
+    with open(os.path.join(os.path.dirname(HERE), "BASELINE.json")) as f:
+        return json.load(f)["reference_path"]
+
+
+REF = os.path.join(reference_dir(), "extensions")
 
 EXTS = {
     "sgutilslib": dict(dir="sgutils", sources=["sg.cu"], fast_math=True),
@@ -76,37 +83,16 @@ def build_one(name):
     return so
 
 
-WRAPPERS = {  # module name under oracle/_ref/pyc -> reference file
-    "ref_sgutils": "/root/reference/extensions/sgutils/sgutils.py",
-    "ref_utils": "/root/reference/extensions/utils/utils.py",
-    "ref_mvpraymarch": "/root/reference/extensions/mvpraymarch/mvpraymarch.py",
-    "ref_render_gsplat": "/root/reference/ca_code/utils/render_gsplat.py",
-}
-
-
-def build_wrappers():
-    """py_compile the reference's L1 wrappers (unchanged) into oracle/_ref/pyc/<name>.pyc."""
-    import py_compile
-
-    out = os.path.join(OUT, "pyc")
-    os.makedirs(out, exist_ok=True)
-    done = []
-    for name, src in WRAPPERS.items():
-        if os.path.exists(src):
-            done.append(py_compile.compile(src, cfile=os.path.join(out, name + ".pyc"), doraise=True))
-    return done
-
-
 def build(names=None):
     if not os.path.isdir(REF):
-        return []  # GPU box: use the prebuilt files
+        sys.stderr.write("oracle/build_ref.py: no reference checkout at %s (set GOLIATH_REFERENCE): the reference's "
+                         "extensions are not built; bench.py --ext-compare and the reference arms of the MVP configs, and "
+                         "tests/golden/make_ref_kernels_golden.py need them\n" % os.path.dirname(REF))
+        return []
     names = names or list(EXTS)
     with ThreadPoolExecutor(max_workers=3) as ex:
-        return list(ex.map(build_one, names)) + build_wrappers()
+        return list(ex.map(build_one, names))
 
 
 if __name__ == "__main__":
-    if sys.argv[1:] == ["wrappers"]:
-        print(build_wrappers())
-    else:
-        print(build(sys.argv[1:] or None))
+    print(build(sys.argv[1:] or None))

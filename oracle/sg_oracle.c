@@ -2,8 +2,8 @@
  * oracle/sg_oracle.c — CPU restatement of the spherical-Gaussian specular shade
  * (reference extensions/sgutils/sg.cu:27-76 forward, :78-175 backward).
  *
- * TEST INFRASTRUCTURE ONLY (see oracle/README.md).  Pinned on the GPU box against the reference's
- * own kernels rebuilt from /root/reference into oracle/_ref/sgutilslib (tests/test_sg_gpu.py);
+ * TEST INFRASTRUCTURE ONLY (see oracle/README.md).  Pinned on the GPU against recorded outputs of the
+ * reference's own kernels rebuilt into oracle/_ref/sgutilslib (tests/golden/ref_kernels_sg.npz);
  * the reference ships no CPU kernel and no test vectors for this op (SURVEY.md §4).
  *
  * Per (batch n, Gaussian d):  integral[n,d,:] = sum_{l < n_lights[n]} light_values[n,l,:] * w

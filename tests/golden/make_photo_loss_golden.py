@@ -32,7 +32,7 @@ def main():
     import ca_code.loss as L
 
     th.manual_seed(226)
-    B, H, W = 4, 45, 70                      # not multiples of the 32-pixel tiles; image wider than tall
+    B, H, W = 4, 45, 56                      # not multiples of the 32-pixel tiles; image wider than tall
     cams = ["400870", "400871", "410001", "400872"]     # identity, colour, GREY ("41..."), colour
     cal = CalV5(cameras=cams, identity_camera="400870").double().eval()   # eval: no lr-scale gradient hook (color_cal.py:239-240)
     with th.no_grad():

@@ -1,153 +1,66 @@
-"""Boundary proof (SURVEY.md section 8b): the REFERENCE's own L1 Python wrappers — extensions/sgutils/sgutils.py,
-extensions/utils/utils.py, extensions/mvpraymarch/mvpraymarch.py, ca_code/utils/render_gsplat.py — run UNCHANGED over
-`goliath_b200.install_dropins()`.
-
-The wrappers are loaded as sourceless bytecode from oracle/_ref/pyc/*.pyc (byte-compiled from /root/reference by
-oracle/build_ref.py in the build container; compiled artefacts like oracle/_ref/*.so, git-ignored, shipped to the GPU
-box; no reference source enters the repo).  CPU leg: the import binds to our modules and a CPU tensor pushed through the
-reference's autograd.Function reaches our C-ABI shim (it raises our no-CPU-fallback error).  GPU leg: results of the
-reference wrappers over our kernels against the CPU oracle."""
-import importlib.machinery
-import importlib.util
+"""CPU: goliath_b200.install_dropins() against the interface the reference's own Python wrappers expect —
+extensions/sgutils/sgutils.py, extensions/utils/utils.py, extensions/mvpraymarch/mvpraymarch.py and
+ca_code/utils/render_gsplat.py.  That interface (imported names, every call into an extension module with its
+positional count and keywords, the argument names of the public functions) is stored as data in
+tests/golden/reference_interface.json, written by tests/golden/make_reference_interface_golden.py."""
+import importlib
+import inspect
+import json
 import os
 import sys
 
-import numpy as np
 import pytest
 import torch
 
-from util import assert_close, small_scene, t2n
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PYC = os.path.join(ROOT, "oracle", "_ref", "pyc")
+IFACE = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_interface.json")))
+OURS = {"extensions/sgutils/sgutils.py": "goliath_b200.sgutils", "extensions/utils/utils.py": "goliath_b200.utils",
+        "extensions/mvpraymarch/mvpraymarch.py": "goliath_b200.mvpraymarch"}
 
 
-def _ref_wrapper(name):
-    path = os.path.join(PYC, name + ".pyc")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/pyc/%s.pyc not built (oracle/build_ref.py needs /root/reference)" % name)
-    import goliath_b200
-
-    goliath_b200.install_dropins()
-    loader = importlib.machinery.SourcelessFileLoader(name, path)
-    spec = importlib.util.spec_from_loader(name, loader)
-    mod = importlib.util.module_from_spec(spec)
-    loader.exec_module(mod)
-    return mod
+def _calls():
+    return [c for w in IFACE.values() for c in w["calls"]]
 
 
 def test_reference_wrappers_bind_to_our_modules():
     import goliath_b200
-    from goliath_b200 import gsplat, mvpraymarchlib, sgutilslib, utilslib
 
-    sg, ut, mv, rg = (_ref_wrapper(n) for n in ("ref_sgutils", "ref_utils", "ref_mvpraymarch", "ref_render_gsplat"))
-    assert sg.sgutilslib is sgutilslib and ut.utilslib is utilslib and mv.mvpraymarchlib is mvpraymarchlib
-    assert rg.project_gaussians is gsplat.project_gaussians and rg.rasterize_gaussians is gsplat.rasterize_gaussians
-    assert sys.modules["gsplat"] is gsplat
+    goliath_b200.install_dropins()
+    imported = {n for w in IFACE.values() for n in w["imports"]}
+    assert imported == {"sgutilslib", "utilslib", "mvpraymarchlib", "gsplat"}
+    for name in imported:  # what the wrappers' `import X` / `from X import ...` now resolve to
+        assert importlib.import_module(name) is importlib.import_module("goliath_b200." + name), name
+    assert sys.modules["gsplat"] is importlib.import_module("goliath_b200.gsplat")
+    gsplat = importlib.import_module("gsplat")
+    for w in IFACE.values():
+        for n in w["imported_names"]:
+            assert callable(getattr(gsplat, n)), n
+    # every call the wrappers make into an extension module binds to the drop-in's signature
+    for c in _calls():
+        fn = getattr(importlib.import_module(c["module"]), c["function"])
+        inspect.signature(fn).bind(*([None] * c["positional"]), **{k: None for k in c["keywords"]})
+    # our mirrors of the wrappers' public functions take the same argument names
+    for path, mod in OURS.items():
+        for fname, names in IFACE[path]["functions"].items():
+            ours = getattr(importlib.import_module(mod), fname)
+            assert list(inspect.signature(ours).parameters) == names, (path, fname)
     # render_raymarcher.py:59 introspects the Python function's co_varnames: it must stay a Python function with them
-    names = mv.mvpraymarch.__code__.co_varnames
+    from goliath_b200.mvpraymarch import mvpraymarch
+    names = mvpraymarch.__code__.co_varnames
     assert {"raypos", "raydir", "stepsize", "tminmax", "primtransf", "template", "warp", "usebvh", "fadescale"} <= set(names)
-    from goliath_b200.mvpraymarch import mvpraymarch as ours
-    assert set(names[:mv.mvpraymarch.__code__.co_argcount]) == set(ours.__code__.co_varnames[:ours.__code__.co_argcount])
+    assert set(names[:mvpraymarch.__code__.co_argcount]) == set(IFACE["extensions/mvpraymarch/mvpraymarch.py"]["functions"]["mvpraymarch"])
 
 
 def test_reference_wrappers_reach_our_abi_on_cpu_tensors():
-    """No GPU here: a CPU tensor through the reference's own Function must arrive at our shim, which refuses it."""
-    sg, ut, rg = _ref_wrapper("ref_sgutils"), _ref_wrapper("ref_utils"), _ref_wrapper("ref_render_gsplat")
+    """No GPU here: each call the reference's wrappers make into sgutilslib / utilslib / mvpraymarchlib, made with CPU
+    tensors, must arrive at our shim, which refuses it (build_tree: a path the reference cannot run either)."""
+    import goliath_b200
+
+    goliath_b200.install_dropins()
     t = torch.zeros(1, 4, 3)
-    with pytest.raises(RuntimeError, match="CUDA"):
-        sg.evaluate_gaussian(t, t[..., 0] + 0.1, t, t, t, torch.ones(1, dtype=torch.int32))
-    with pytest.raises(RuntimeError, match="CUDA"):
-        # (the reference's wrapper asserts .is_contiguous() on pixelcoords, utils.py:29-30: a (W, H) tuple never gets through it)
-        ut.compute_raydirs(torch.zeros(1, 3), torch.eye(3)[None], torch.ones(1, 2), torch.zeros(1, 2),
-                           torch.zeros(1, 8, 8, 2), 1.0)
-    with pytest.raises(RuntimeError, match="CUDA"):
-        rg.render(16, 16, 10.0, 10.0, 8.0, 8.0, torch.eye(4)[:3].contiguous(), torch.zeros(4, 3),
-                  torch.tensor([[1.0, 0.0, 0.0, 0.0]] * 4), torch.ones(4, 3), torch.ones(4, 1), torch.ones(4, 3))
-
-
-@pytest.mark.gpu
-def test_reference_sgutils_wrapper_vs_oracle(orc, cuda):
-    from test_oracle_sg import make
-
-    sg = _ref_wrapper("ref_sgutils")
-    dirs, sig, lv, lp, pp, nl = make(N=2, D=3000, L=12, seed=77)
-    c = lambda t: t.to(cuda)
-    dd, ss, ll = c(dirs).requires_grad_(), c(sig).requires_grad_(), c(lv).requires_grad_()
-    out = sg.evaluate_gaussian(dd, ss, ll, c(lp), c(pp), c(nl), w_type=0, normalize_lobe_dirs=False)
-    ref = orc.sg_fwd(dirs.numpy(), sig.numpy(), lv.numpy(), lp.numpy(), pp.numpy(), nl.numpy(), 0)
-    assert_close(t2n(out), ref, rtol=1e-3, atol=1e-4 * float(np.abs(ref).max()), frac=0.999, what="integral")
-    g = torch.randn(out.shape, generator=torch.Generator().manual_seed(2))
-    out.backward(c(g))
-    gd, gs, gl = orc.sg_bwd(dirs.numpy(), sig.numpy(), lv.numpy(), lp.numpy(), pp.numpy(), nl.numpy(), g.numpy(), 0)
-    assert_close(t2n(ss.grad), gs, rtol=2e-3, atol=1e-4 * float(np.abs(gs).max()), frac=0.999, what="grad_sigmas")
-    assert_close(t2n(dd.grad), gd, rtol=2e-3, atol=1e-4 * float(np.abs(gd).max()), frac=0.999, what="grad_dirs")
-    assert_close(t2n(ll.grad), gl, rtol=1e-3, atol=1e-4 * float(np.abs(gl).max()), what="grad_light_values")
-
-
-@pytest.mark.gpu
-def test_reference_raymarch_wrappers_vs_oracle(orc, cuda):
-    from goliath_b200 import synthetic
-
-    ut, mv = _ref_wrapper("ref_utils"), _ref_wrapper("ref_mvpraymarch")
-    s = synthetic.mvp_scene(N=2, side=8, img_h=64, img_w=48)
-    t = {k: (v.to(cuda) if torch.is_tensor(v) else v) for k, v in s.items()}
-    px, py = torch.meshgrid(torch.arange(48.0), torch.arange(64.0), indexing="xy")
-    pix = (torch.stack([px, py], -1)[None].repeat(2, 1, 1, 1) + 0.5).contiguous().to(cuda)
-    raypos, raydir, tminmax = ut.compute_raydirs(t["viewpos"], t["viewrot"], t["focal"], t["princpt"], pix, t["volradius"])
-    n = lambda x: x.detach().cpu().numpy()
-    o = orc.raydirs_fwd(n(s["viewpos"]), n(s["viewrot"]), n(s["focal"]), n(s["princpt"]), n(pix), 1.0)
-    assert_close(t2n(raydir), o[1], rtol=1e-6, what="raydir")
-    assert_close(t2n(tminmax), o[2], rtol=1e-5, what="tminmax")
-    step = 0.02
-    pp, pr, ps = t["primpos"].requires_grad_(), t["primrot"].requires_grad_(), t["primscale"].requires_grad_()
-    tpl = t["template"].requires_grad_()
-    out = mv.mvpraymarch(raypos, raydir, step, tminmax, (pp, pr, ps), tpl, None, algo=0, fadescale=8.0, fadeexp=8.0)
-    o_rgba, o_sat, _ = orc.raymarch_fwd(n(raypos), n(raydir), step, n(tminmax), n(pp), n(pr), n(ps), n(tpl), None, algo=0)
-    assert (o_rgba[..., 3] > 0.05).mean() > 0.05
-    assert_close(t2n(out), o_rgba, rtol=2e-4, atol=2e-5, frac=0.999, what="rayrgba")
-    g = torch.randn(out.shape, generator=torch.Generator().manual_seed(5)).to(cuda)
-    out.backward(g)
-    gp, gr, gs, gt, _ = orc.raymarch_bwd(n(raypos), n(raydir), step, n(tminmax), n(pp), n(pr), n(ps), n(tpl), None, o_sat,
-                                         n(g), algo=0)
-    assert_close(t2n(tpl.grad), gt, rtol=1e-3, atol=1e-4 * np.abs(gt).max(), frac=0.995, what="grad_template")
-    assert_close(t2n(pp.grad), gp, rtol=1e-3, atol=2e-3 * np.abs(gp).max(), frac=0.995, what="grad_primpos")
-
-
-@pytest.mark.gpu
-def test_reference_render_gsplat_wrapper_vs_oracle(orc, cuda):
-    rg = _ref_wrapper("ref_render_gsplat")
-    s = small_scene(G=3000, img_h=96, img_w=80)
-    mult = 12.0
-    d = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(cuda)
-    H, W = s["img_h"], s["img_w"]
-    leaves = dict(primpos=d(s["means3d"]).requires_grad_(), primqvec=d(s["quats"]).requires_grad_(),
-                  primscale=d(s["scales"] * np.float32(mult)).requires_grad_(), opacity=d(s["opacity"]).requires_grad_(),
-                  colors=d(s["colors"]).requires_grad_())
-    o = rg.render(W, H, s["fx"], s["fy"], s["cx"], s["cy"], d(s["viewmat"]), leaves["primpos"], leaves["primqvec"],
-                  leaves["primscale"], leaves["opacity"], leaves["colors"], return_depth=True)
-    p = orc.project_fwd(s["means3d"], s["scales"] * np.float32(mult), 1.0, s["quats"], s["viewmat"], s["fx"], s["fy"],
-                        s["cx"], s["cy"], H, W, 16, 0.1)
-    b = orc.bin_and_sort(p["xys"], p["depths"], p["radii"], p["num_tiles_hit"], H, W, 16)
-    opac = (s["opacity"][:, 0] * p["compensation"]).astype(np.float32)
-    z3 = np.zeros(3, np.float32)
-    img, Ts, fi = orc.rasterize_fwd(H, W, 16, b["gaussian_ids_sorted"], b["tile_bins"], p["xys"], p["conics"], s["colors"],
-                                    opac, z3)
-    dep, _, _ = orc.rasterize_fwd(H, W, 16, b["gaussian_ids_sorted"], b["tile_bins"], p["xys"], p["conics"],
-                                  np.repeat(p["depths"][:, None], 3, 1), opac, z3)
-    assert np.array_equal(t2n(o["radii"]), p["radii"])
-    assert_close(t2n(o["render"]), np.transpose(img, (2, 0, 1)), rtol=1e-4, atol=2e-5, frac=0.9995, what="render")
-    assert_close(t2n(o["final_T"][0]), Ts, rtol=1e-4, atol=2e-6, frac=0.9995, what="final_T")
-    assert_close(t2n(o["depth"][0]), dep[..., 0], rtol=1e-4, atol=2e-2, frac=0.9995, what="depth")
-    # gradient of sum(render) through the reference's own autograd glue (opacity * compensation in PyTorch)
-    o["render"].sum().backward()
-    g = orc.rasterize_bwd(H, W, 16, b["gaussian_ids_sorted"], b["tile_bins"], p["xys"], p["conics"], s["colors"], opac, z3,
-                          Ts, fi, np.ones((H, W, 3), np.float32), np.zeros((H, W), np.float32))
-    pb = orc.project_bwd(s["means3d"], s["scales"] * np.float32(mult), 1.0, s["quats"], s["viewmat"], s["fx"], s["fy"],
-                         p["cov3d"], p["radii"], p["conics"], p["compensation"], g[0], np.zeros(len(opac), np.float32), g[1],
-                         g[3][:, 0] * s["opacity"][:, 0])
-    assert_close(t2n(leaves["colors"].grad), g[2], rtol=1e-4, atol=1e-5 * np.abs(g[2]).max(), frac=0.999, what="v_colors")
-    want_op = (g[3][:, 0] * p["compensation"])[:, None]
-    assert_close(t2n(leaves["opacity"].grad), want_op, rtol=1e-4, atol=1e-5 * np.abs(want_op).max(), frac=0.999, what="v_opacity")
-    assert_close(t2n(leaves["primpos"].grad), pb["v_mean3d"], rtol=1e-3, atol=1e-4 * np.abs(pb["v_mean3d"]).max(), frac=0.999,
-                 what="v_mean3d")
+    for c in _calls():
+        if c["module"] == "gsplat":
+            continue
+        fn = getattr(importlib.import_module(c["module"]), c["function"])
+        with pytest.raises(RuntimeError, match="CUDA" if c["function"] != "build_tree" else "reference"):
+            fn(*([t] * c["positional"]), **{k: t for k in c["keywords"]})

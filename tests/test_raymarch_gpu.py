@@ -2,30 +2,20 @@
 surface (goliath_b200.utils.compute_raydirs, goliath_b200.mvpraymarch.mvpraymarch) against
   * the CPU oracle (oracle/raymarch_oracle.c),
   * the reference's PyTorch-oracle fixtures (tests/golden/raymarch_pytorch_ref.npz),
-  * the reference's own kernels rebuilt for sm_100a into oracle/_ref (utilslib.so, mvpraymarchlib.so)."""
-import importlib.util
+  * the outputs of the reference's own kernels rebuilt for sm_100a (utilslib, mvpraymarchlib) on the same inputs
+    (tests/golden/ref_kernels_{mvp,raymarch}.npz, written by tests/golden/make_ref_kernels_golden.py)."""
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from goliath_b200 import synthetic
-from util import assert_close, t2n
+from util import (MARCH_KEYS, MARCH_SCENE, MARCH_STEP, assert_close, load_ref_golden, march_grad, march_inputs,
+                  mvp_scene, raydirs_pixels, ref_pair, t2n)
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden", "raymarch_pytorch_ref.npz")
-
-
-def _ref(name):
-    so = os.path.join(ROOT, "oracle", "_ref", name + ".so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref/%s.so not built (needs /root/reference at build time)" % name)
-    spec = importlib.util.spec_from_file_location(name, so)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    return m
 
 
 @pytest.fixture(params=["legacy", "queue"], autouse=True)
@@ -40,12 +30,6 @@ def raymarch_mode(request):
     L.gb_set_raymarch_mode(before)
 
 
-def _scene(dev, **kw):
-    s = synthetic.mvp_scene(**kw)
-    t = {k: (v.to(dev) if torch.is_tensor(v) else v) for k, v in s.items()}
-    return s, t
-
-
 def _rays(t):
     from goliath_b200.utils import compute_raydirs
 
@@ -53,7 +37,7 @@ def _rays(t):
 
 
 def test_raydirs_vs_oracle_and_reference(orc, cuda):
-    s, t = _scene(cuda, N=3, img_h=37, img_w=45)
+    s, t = mvp_scene(cuda, N=3, img_h=37, img_w=45)
     raypos, raydir, tminmax = _rays(t)
     n = lambda x: x.numpy()
     o = orc.raydirs_fwd(n(s["viewpos"]), n(s["viewrot"]), n(s["focal"]), n(s["princpt"]), None, 1.0, H=37, W=45)
@@ -62,42 +46,28 @@ def test_raydirs_vs_oracle_and_reference(orc, cuda):
     assert_close(t2n(tminmax), o[2], rtol=1e-5, what="tminmax")
     # explicit pixel coordinates
     from goliath_b200.utils import compute_raydirs
-    px, py = torch.meshgrid(torch.arange(45.0), torch.arange(37.0), indexing="xy")
-    pix = (torch.stack([px, py], -1)[None].repeat(3, 1, 1, 1) + 0.5).contiguous().to(cuda)
+    pix = raydirs_pixels(3, 37, 45)
+    ref = load_ref_golden("mvp", "raydirs_", [s["viewpos"], s["viewrot"], s["focal"], s["princpt"], pix])
+    pix = pix.to(cuda)
     r2 = compute_raydirs(t["viewpos"], t["viewrot"], t["focal"], t["princpt"], pix, 1.0)
     o2 = orc.raydirs_fwd(n(s["viewpos"]), n(s["viewrot"]), n(s["focal"]), n(s["princpt"]), t2n(pix), 1.0)
     assert_close(t2n(r2[1]), o2[1], rtol=1e-6, what="raydir(pix)")
-    ref = _ref("utilslib")
-    rr = [torch.empty_like(x) for x in r2]
-    ref.compute_raydirs_forward(t["viewpos"], t["viewrot"], t["focal"], t["princpt"], pix, 45, 37, 1.0, *rr)
-    torch.cuda.synchronize()
-    for a, b, name in zip(r2, rr, ("raypos", "raydir", "tminmax")):
-        assert torch.equal(a, b), "%s not bit-identical to the reference kernel" % name
+    for a, name in zip(r2, ("raypos", "raydir", "tminmax")):
+        assert np.array_equal(t2n(a), ref[name]), "%s not bit-identical to the reference kernel" % name
 
 
 def test_compute_aabb_vs_oracle_and_reference(orc, cuda):
     from goliath_b200.mvpraymarch import build_accel
 
     for side in (4, 5, 8):  # K = 16, 25 (not a power of two), 64
-        s, t = _scene(cuda, N=2, side=side)
+        s, t = mvp_scene(cuda, N=2, side=side)
         sid, ch, aabb = build_accel((t["primpos"], t["primrot"], t["primscale"]), 0, fixedorder=True)
         o = orc.compute_aabb_fixedorder(s["primpos"].numpy(), s["primrot"].numpy(), s["primscale"].numpy())
         assert_close(t2n(aabb), o, rtol=1e-5, what="nodeaabb K=%d" % (side * side))
         K = side * side
         assert np.array_equal(t2n(sid), np.tile(np.arange(K, dtype=np.int32), (2, 1)))
-    ref = _ref("mvpraymarchlib")
-    from goliath_b200.mvpraymarch import _fixedorder_topology
-    sid, ch, par = _fixedorder_topology(2, 64, cuda)
-    ra = torch.empty_like(aabb)
-    ref.compute_aabb(t["primpos"], t["primrot"], t["primscale"], sid, ch, par, ra, 0)
-    torch.cuda.synchronize()
-    assert torch.equal(ra, aabb), "nodeaabb not bit-identical to the reference kernel"
-
-
-def _march_inputs(dev, algo, **kw):
-    s, t = _scene(dev, with_warp=(algo == 1), **kw)
-    raypos, raydir, tminmax = _rays(t)
-    return s, t, raypos, raydir, tminmax
+    ref = load_ref_golden("mvp", "aabb_", [s["primpos"], s["primrot"], s["primscale"]])
+    assert np.array_equal(t2n(aabb), ref["nodeaabb"]), "nodeaabb not bit-identical to the reference kernel"
 
 
 @pytest.mark.parametrize("algo", [0, 1])
@@ -106,7 +76,7 @@ def test_raymarch_vs_oracle(orc, cuda, algo, cfg):
     """forward + backward against the CPU oracle; the second config is dense enough to saturate rays and has K=25."""
     from goliath_b200.mvpraymarch import mvpraymarch
 
-    s, t, raypos, raydir, tminmax = _march_inputs(cuda, algo, **cfg)
+    s, t, raypos, raydir, tminmax = march_inputs(cuda, algo, **cfg)
     step = 0.02
     pp, pr, ps = t["primpos"].requires_grad_(), t["primrot"].requires_grad_(), t["primscale"].requires_grad_()
     tpl = t["template"].requires_grad_()
@@ -155,52 +125,52 @@ def test_raymarch_vs_reference_pytorch_fixture(cuda, tag, algo):
 
 @pytest.mark.parametrize("algo", [0, 1])
 def test_raymarch_vs_reference_kernels(cuda, algo):
-    """Same tensors through the reference's mvpraymarchlib (rebuilt, -use_fast_math) and through ours."""
-    ref = _ref("mvpraymarchlib")
+    """Same tensors as the reference's mvpraymarchlib (rebuilt, -use_fast_math) was run on, through ours; the backward
+    of both reads the reference's forward outputs.  The template / warp gradients are a fixed sample.  The fixture's
+    input digest covers the seeded scene and output gradient, not the rays: they come from our compute_raydirs, which
+    test_raydirs_vs_oracle_and_reference pins bit for bit to the reference kernel."""
     from goliath_b200 import mvpraymarchlib as ours
-    from goliath_b200.mvpraymarch import _fixedorder_topology, build_accel
+    from goliath_b200.mvpraymarch import build_accel
 
-    s, t, raypos, raydir, tminmax = _march_inputs(cuda, algo, N=2, side=12, T=(4, 8, 8), img_h=96, img_w=72, density=150.0)
+    s, t, raypos, raydir, tminmax = march_inputs(cuda, algo, **MARCH_SCENE)
     N, H, W = raypos.shape[:3]
-    K = t["primpos"].shape[1]
+    g = march_grad((N, H, W))
+    ref = load_ref_golden("raymarch", "algo%d_" % algo, [s[k] for k in MARCH_KEYS if k in s] + [g])
     sid, ch, aabb = build_accel((t["primpos"], t["primrot"], t["primscale"]), algo, fixedorder=True)
     warp = t["warp"] if algo == 1 else None
-    step = 0.01
-    res = []
-    for lib in (ref, ours):
-        rgba = torch.empty(N, H, W, 4, device=cuda)
-        sat = torch.full((N, H, W, 3), -1.0, device=cuda)
-        lib.raymarch_forward(raypos, raydir, step, tminmax, sid, ch, aabb, t["primpos"], t["primrot"], t["primscale"],
-                             t["template"], warp, rgba, sat, None, None, algo, False, 512, True, True, 8.0, 8.0, 0, 0.99, 3,
-                             8, 16)
-        torch.cuda.synchronize()
-        res.append((rgba, sat))
-    r, o = res
-    assert (r[0][..., 3] > 0.05).float().mean() > 0.05
-    same = (r[0] == o[0]).float().mean().item()
-    assert_close(t2n(o[0]), t2n(r[0]), rtol=1e-5, atol=1e-6, frac=0.9999, what="rayrgba vs reference kernel")
+    step = MARCH_STEP
+    rgba = torch.empty(N, H, W, 4, device=cuda)
+    sat = torch.full((N, H, W, 3), -1.0, device=cuda)
+    ours.raymarch_forward(raypos, raydir, step, tminmax, sid, ch, aabb, t["primpos"], t["primrot"], t["primscale"],
+                          t["template"], warp, rgba, sat, None, None, algo, False, 512, True, True, 8.0, 8.0, 0, 0.99, 3,
+                          8, 16)
+    torch.cuda.synchronize()
+    r_rgba, r_sat = ref["rayrgba"], ref["raysat"]
+    assert (r_rgba[..., 3] > 0.05).mean() > 0.05
+    same = (t2n(rgba) == r_rgba).mean()
+    assert_close(t2n(rgba), r_rgba, rtol=1e-5, atol=1e-6, frac=0.9999, what="rayrgba vs reference kernel")
     assert same > 0.99, "only %.4f of rayrgba values bit-identical to the reference kernel" % same
-    assert_close(t2n(o[1]), t2n(r[1]), rtol=1e-5, atol=1e-6, frac=0.9999, what="raysat vs reference kernel")
-    g = torch.randn(N, H, W, 4, generator=torch.Generator().manual_seed(11)).to(cuda)
-    grads = []
-    for lib in (ref, ours):
-        gp, gr, gs = torch.zeros_like(t["primpos"]), torch.zeros_like(t["primrot"]), torch.zeros_like(t["primscale"])
-        gt = torch.zeros_like(t["template"])
-        gw = torch.zeros_like(warp) if warp is not None else None
-        lib.raymarch_backward(raypos, raydir, step, tminmax, sid, ch, aabb, t["primpos"], gp, t["primrot"], gr,
-                              t["primscale"], gs, t["template"], gt, warp, gw, r[0], g, r[1], None, algo, False, 512, True,
-                              True, 8.0, 8.0, 0, 0.99, 3, 8, 16)
-        torch.cuda.synchronize()
-        grads.append((gp, gr, gs, gt) + ((gw,) if gw is not None else ()))
-    for name, x, y in zip(("grad_primpos", "grad_primrot", "grad_primscale", "grad_template", "grad_warp"), grads[1], grads[0]):
-        y = t2n(y)
-        assert_close(t2n(x), y, rtol=1e-4, atol=1e-5 * np.abs(y).max(), frac=0.9995, what=name + " vs reference kernel")
+    assert_close(t2n(sat), r_sat, rtol=1e-5, atol=1e-6, frac=0.9999, what="raysat vs reference kernel")
+    gp, gr, gs = torch.zeros_like(t["primpos"]), torch.zeros_like(t["primrot"]), torch.zeros_like(t["primscale"])
+    gt = torch.zeros_like(t["template"])
+    gw = torch.zeros_like(warp) if warp is not None else None
+    ours.raymarch_backward(raypos, raydir, step, tminmax, sid, ch, aabb, t["primpos"], gp, t["primrot"], gr,
+                           t["primscale"], gs, t["template"], gt, warp, gw, torch.from_numpy(r_rgba).to(cuda), g.to(cuda),
+                           torch.from_numpy(r_sat).to(cuda), None, algo, False, 512, True, True, 8.0, 8.0, 0, 0.99, 3, 8,
+                           16)
+    torch.cuda.synchronize()
+    for name, t in zip(("grad_primpos", "grad_primrot", "grad_primscale", "grad_template", "grad_warp"),
+                       (gp, gr, gs, gt, gw)):
+        if t is None:
+            continue
+        x, y, absmax = ref_pair(ref, name, t)
+        assert_close(x, y, rtol=1e-4, atol=1e-5 * absmax, frac=0.9995, what=name + " vs reference kernel")
 
 
 def test_shadow_splat_vs_oracle(orc, cuda):
     from goliath_b200.mvpraymarch import mvpraymarch
 
-    s, t, raypos, raydir, tminmax = _march_inputs(cuda, 0, N=1, side=6, img_h=40, img_w=33)
+    s, t, raypos, raydir, tminmax = march_inputs(cuda, 0, N=1, side=6, img_h=40, img_w=33)
     with torch.no_grad():
         out, shadow = mvpraymarch(raypos, raydir, 0.02, tminmax, (t["primpos"], t["primrot"], t["primscale"]), t["template"],
                                   None, with_shadow=True)
