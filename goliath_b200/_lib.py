@@ -38,6 +38,8 @@ SIGNATURES = {
     "gb_map_gaussian_to_intersects_dn": (_i, [_i, _vp, _vp, _vp, _vp, _i, _i, _i, _i64, _vp, _vp, _vp]),
     "gb_sort_intersects_dn": (_i, [_i64, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
     "gb_get_tile_bin_edges_dn": (_i, [_i64, _vp, _vp, _vp, _vp, _vp]),
+    "gb_get_bin_sort_mode": (_i, []),
+    "gb_set_bin_sort_mode": (None, [_i]),
     "gb_get_tile_sort_mode": (_i, []),
     "gb_set_tile_sort_mode": (None, [_i]),
     "gb_get_rank_sort_mode": (_i, []),

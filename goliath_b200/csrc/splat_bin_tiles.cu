@@ -3,14 +3,29 @@
 // Produces exactly what the key sort of csrc/splat_bin.cu produces for the fused render — per-tile
 // [first,last) bins, the Gaussian ids of every tile in front-to-back order (ties: ascending id), and the
 // packed blend records — i.e. the work gsplat 0.1.11 does in bin_and_sort_gaussians (called from
-// rasterize_gaussians, call sites ca_code/utils/render_gsplat.py:65-78,90-104), but without ever sorting
-// the I (tile, depth) intersection keys:
+// rasterize_gaussians, call sites ca_code/utils/render_gsplat.py:65-78,90-104), but without a global sort of
+// the I (tile, depth) intersection keys.  Two orderings, same outputs (gb_set_bin_sort_mode, GOLIATH_B200_BINSORT):
 //
-//   1. depth_keys_kernel     G threads: depth bits -> 32-bit sort key, digit-0 histogram, and the per-tile
-//                            intersection COUNT of every visible Gaussian.  Counts are privatised per CTA in
-//                            shared memory and flushed with one RED per (CTA, non-empty tile): the hot tiles
-//                            of a head scene take ~2000 hits each, which serialise on the L2 atomic unit when
-//                            issued one by one (measured: 118 us with one global RED per pair, 8 us privatised).
+// TILE (default): bucket the pairs, sort each tile's short list on chip.
+//   1. depth_keys_kernel<., false>   G threads: per-tile intersection COUNT of every visible Gaussian, and the min /
+//                            max of the visible depth keys (sync[4..5]).  Counts are privatised per CTA in shared
+//                            memory and flushed with one RED per (CTA, non-empty tile): the hot tiles of a head scene
+//                            take ~2000 hits each, which serialise on the L2 atomic unit when issued one by one
+//                            (measured: 118 us with one global RED per pair, 8 us privatised).
+//   2. tile_scan_kernel + gb_tile_order / gb_tile_schedule, as below.
+//   3. tile_scatter_kernel<true>     G threads: every (Gaussian, tile) pair writes the Gaussian's 32-bit depth key into
+//                            its slot of tile_ranks and its id into the same slot of gids_sorted (slots claimed per
+//                            CTA, order inside a bucket arbitrary); the 48-byte record goes to a table indexed BY ID.
+//   4. tile_pair_sort_kernel one CTA per tile, longest first: composite (key - min key) << 32 | id — unique, and
+//                            ordered as the key sort orders the tile (depth bits, ties by ascending id) — LSD radix
+//                            sorted in shared memory over the KEY digits that vary inside the tile, then each run of
+//                            equal keys put in id order (all digits when a run is long); sorted ids written back.  A list longer than kPairCap sorts in the
+//                            tile's own slots of the records output (48 B per slot, 16 B used), written only by 5.
+//   5. gather_records_kernel grid-wide: records[i] = table[gids_sorted[i]] (rec_colors_kernel first with late colours).
+//   Workspace per intersection slot stays 4 bytes; no depth ranks, no cooperative launch, no per-tile G-bit bitmap.
+//
+// RANK: depth-rank the G Gaussians once, then order each tile's ranks with a bitmap.
+//   1. depth_keys_kernel<., true>    as above, plus the key array and the digit-0 histogram of the rank sort.
 //   2. rank_scatter_kernel   x4: stable LSD radix sort of the G depth keys (8-bit digits).  One kernel per
 //                            pass: a CTA derives its own scatter bases from the per-CTA histogram table
 //                            (column prefix read from L2) and accumulates the NEXT pass's table with global
@@ -32,8 +47,12 @@
 //                            popcount prefix -> sorted ranks -> (Gaussian id, record copied from the by-rank
 //                            table with monotonically increasing addresses), written linearly.
 //
+//   (2b is the default form of 2, one cooperative kernel; 5b the default form of 5, bitmap sort + grid-wide gather.)
+//   gb_bin_tiles_ranked always takes this path: its blend reads records by depth rank.
+//
 // Integer/byte work with a BIT-EXACT contract: gids_sorted, tile_bins and records are identical to the
-// key-sort path's (tests/test_splat_gpu.py::test_bin_tiles_matches_key_sort).
+// key-sort path's under either ordering (tests/test_splat_gpu.py::test_bin_tiles_matches_key_sort,
+// tests/test_bin_tiles_tilesort_gpu.py).
 #include <stdlib.h>
 #include <string.h>
 
@@ -107,8 +126,9 @@ __device__ __forceinline__ void tile_bbox(float cx, float cy, float radius, int 
 // smem_tiles = T: per-CTA counters in dynamic shared memory; 0: global atomics (more tiles than fit).
 // A CTA covers one tile of the rank sort (kTileKeys keys) with kGaussBlock threads: few fat CTAs keep the number
 // of counter flushes low, many threads per CTA keep enough loads in flight (the kernel is latency-bound).
+// kRank = false (per-tile sort path): no key array and no digit-0 histogram, only the tile counts and sync[4..5].
 constexpr int kGaussBlock = 1024;
-template <int kTileKeys>
+template <int kTileKeys, bool kRank>
 __global__ void __launch_bounds__(kGaussBlock) depth_keys_kernel(int G, const float2* __restrict__ xys,
                                                                  const float* __restrict__ depths,
                                                                  const int* __restrict__ radii, int tbx, int tby,
@@ -156,8 +176,10 @@ __global__ void __launch_bounds__(kGaussBlock) depth_keys_kernel(int G, const fl
   for (int j = 0; j < kItems; ++j) {
     const int i = base + j * kGaussBlock + threadIdx.x;
     if (i >= G) continue;
-    keys[i] = k[j];
-    atomicAdd(&s_hist[k[j] & 0xffu], 1u);
+    if (kRank) {
+      keys[i] = k[j];
+      atomicAdd(&s_hist[k[j] & 0xffu], 1u);
+    }
     if (r[j] > 0) {
       int x0, y0, x1, y1;
       tile_bbox(c[j].x, c[j].y, (float)r[j], tbx, tby, block_width, x0, y0, x1, y1);
@@ -173,7 +195,7 @@ __global__ void __launch_bounds__(kGaussBlock) depth_keys_kernel(int G, const fl
     atomicOr(key_bits, s_or); atomicOr(key_bits + 1, s_orc);
     atomicMax(key_bits + 4, s_max); atomicMax(key_bits + 5, s_maxc);  // [4] = max visible key, [5] = ~min visible key
   }
-  if (threadIdx.x < kRadix) hist0[(size_t)blockIdx.x * kRadix + threadIdx.x] = s_hist[threadIdx.x];
+  if (kRank && threadIdx.x < kRadix) hist0[(size_t)blockIdx.x * kRadix + threadIdx.x] = s_hist[threadIdx.x];
   for (int t = threadIdx.x; t < smem_tiles; t += kGaussBlock) {
     const int cnt = s_cnt[t];
     if (cnt) atomicAdd(&tile_counts[t], cnt);
@@ -633,20 +655,24 @@ __global__ void __launch_bounds__(1024) tile_scan_kernel(int T, long long cap, c
   }
 }
 
-// ------------------------------------------------------------------ 4. ranks into the tile buckets + by-rank records
+// ------------------------------------------------------------------ 4. pairs into the tile buckets + per-Gaussian records
 // smem_tiles = T: slots claimed per CTA through shared memory (s_cnt | s_base, 2*T ints); 0: one global atomic
 // per (Gaussian, tile).  kGaussBlock threads x kScatItems Gaussians per CTA (see depth_keys_kernel).
+// kById = false (rank path): a slot receives the Gaussian's depth RANK, the record table is indexed by rank.
+// kById = true (per-tile sort path): a slot receives the Gaussian's 32-bit depth key in tile_ranks and its id in the
+// same slot of slot_ids (the gids_sorted output); the record table is indexed by id.
+template <bool kById>
 __global__ void __launch_bounds__(kGaussBlock) tile_scatter_kernel(
     int G, const float2* __restrict__ xys, const int* __restrict__ radii, const int* __restrict__ rank_of,
     const float* __restrict__ conics, const float* __restrict__ colors3, const float* __restrict__ depths,
     const float* __restrict__ opacity, const float* __restrict__ comp, int tbx, int tby, int block_width,
-    long long cap, int smem_tiles, int* __restrict__ cursor, int* __restrict__ tile_ranks,
+    long long cap, int smem_tiles, int* __restrict__ cursor, int* __restrict__ tile_ranks, int* __restrict__ slot_ids,
     float4* __restrict__ rec_by_rank) {
   extern __shared__ int s_cnt[];
   int* s_base = s_cnt + smem_tiles;
   for (int t = threadIdx.x; t < smem_tiles; t += kGaussBlock) s_cnt[t] = 0;
   const int base = blockIdx.x * (kGaussBlock * kScatItems);
-  int rk[kScatItems], r[kScatItems];
+  int rk[kScatItems], r[kScatItems];  // rk: what goes into tile_ranks (rank, or depth key bits when kById)
   float2 c[kScatItems];
 #pragma unroll
   for (int j = 0; j < kScatItems; ++j) {  // all loads first: independent, in flight together
@@ -654,7 +680,8 @@ __global__ void __launch_bounds__(kGaussBlock) tile_scatter_kernel(
     const bool in = i < G;
     r[j] = in ? radii[i] : 0;
     c[j] = in ? xys[i] : make_float2(0.f, 0.f);
-    rk[j] = in ? rank_of[i] : 0;
+    if (kById) rk[j] = in ? __float_as_int(depths[i]) : 0;
+    else rk[j] = in ? rank_of[i] : 0;
   }
   __syncthreads();
   unsigned bx[kScatItems], by[kScatItems];  // x0 | x1 << 16, y0 | y1 << 16 (tile coordinates < 65536)
@@ -667,14 +694,17 @@ __global__ void __launch_bounds__(kGaussBlock) tile_scatter_kernel(
     tile_bbox(c[j].x, c[j].y, (float)r[j], tbx, tby, block_width, x0, y0, x1, y1);
     bx[j] = (unsigned)x0 | ((unsigned)x1 << 16);
     by[j] = (unsigned)y0 | ((unsigned)y1 << 16);
-    gb::pack_record_fused(i, xys, conics, colors3, depths, opacity, comp, rec_by_rank + 3 * (size_t)rk[j]);
+    gb::pack_record_fused(i, xys, conics, colors3, depths, opacity, comp, rec_by_rank + 3 * (size_t)(kById ? i : rk[j]));
     for (int ty = y0; ty < y1; ++ty)
       for (int tx = x0; tx < x1; ++tx) {
         if (smem_tiles) {
           atomicAdd(&s_cnt[ty * tbx + tx], 1);
         } else {
           const int pos = atomicAdd(&cursor[ty * tbx + tx], 1);
-          if ((long long)pos < cap) tile_ranks[pos] = rk[j];
+          if ((long long)pos < cap) {
+            tile_ranks[pos] = rk[j];
+            if (kById) slot_ids[pos] = i;
+          }
         }
       }
   }
@@ -693,7 +723,10 @@ __global__ void __launch_bounds__(kGaussBlock) tile_scatter_kernel(
       for (int tx = x0; tx < x1; ++tx) {
         const int t = ty * tbx + tx;
         const int pos = s_base[t] + atomicAdd(&s_cnt[t], 1);
-        if ((long long)pos < cap) tile_ranks[pos] = rk[j];
+        if ((long long)pos < cap) {
+          tile_ranks[pos] = rk[j];
+          if (kById) slot_ids[pos] = base + j * kGaussBlock + threadIdx.x;
+        }
       }
   }
 }
@@ -812,24 +845,183 @@ __global__ void __launch_bounds__(kSortThreads, 3) tile_sort_kernel(int words, i
   }
 }
 
-// Late colours (gb_bin_tiles_pack_ev with an event): tile_scatter leaves the colour quarter of the by-rank records
+// ------------------------------------------------------------------ 5c. per-tile (depth key, id) sort (default)
+// The tile's slots hold (32-bit depth key, Gaussian id) pairs in arbitrary order.  One CTA per tile, longest first, forms
+// the 64-bit composite (key - min visible key) << 32 | id — unique, and ordered exactly as the key sort orders the
+// tile (depth bits, ties by ascending id) — and radix-sorts it in 8-bit digits (pair_sort_tile: key digits first).  Up to
+// kPairCap pairs live in shared memory; a longer tile sorts in the 48-byte record slots of its own range of the records
+// output (16 B per pair used), which only the record gather writes, later.
+constexpr int kPairThreads = 512;
+constexpr int kPairWarps = kPairThreads / 32;
+constexpr int kPairCap = 6144;  // 2 x 48 KB ping-pong + 16 KB warp histograms = 112 KB: two CTAs per SM
+constexpr size_t kPairSmem = (size_t)2 * kPairCap * 8 + (size_t)kPairWarps * kRadix * 4;
+
+// Stable LSD radix sort of a[0, n) over the 8-bit digits in which `varying` has a bit, ping-ponging between a and b;
+// returns the buffer that holds the result.  Warp w owns the contiguous chunk [w*per, (w+1)*per) and walks it 32 pairs
+// at a time, so "earlier in the buffer" == "earlier warp, or earlier in the same warp's walk": the scatter is stable.
+__device__ __forceinline__ unsigned long long* pair_radix_sort(unsigned long long* a, unsigned long long* b, int n,
+                                                               unsigned long long varying, unsigned* s_hist, int* s_warp) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int per = (n + kPairWarps - 1) / kPairWarps;
+  const int c0 = min(n, warp * per), c1 = min(n, c0 + per);
+  const unsigned lt = (1u << lane) - 1u;
+  unsigned* h = s_hist + warp * kRadix;
+  for (int shift = 0; shift < 64; shift += 8) {
+    if (((varying >> shift) & 0xffull) == 0ull) continue;  // the same digit for every pair: identity pass
+    for (int d = lane; d < kRadix; d += 32) h[d] = 0u;
+    __syncwarp();
+    for (int i = c0 + lane; i < c1; i += 32) atomicAdd(&h[(unsigned)(a[i] >> shift) & 0xffu], 1u);
+    __syncthreads();
+    {  // scatter bases, digit-major then warp: smaller digits anywhere + the same digit in earlier warps
+      const int d = threadIdx.x;
+      unsigned tot = 0u;
+      if (d < kRadix)
+        for (int w = 0; w < kPairWarps; ++w) tot += s_hist[w * kRadix + d];
+      int unused;
+      unsigned run = (unsigned)block_exclusive_scan((int)tot, s_warp, unused);
+      if (d < kRadix)
+        for (int w = 0; w < kPairWarps; ++w) {
+          const unsigned c = s_hist[w * kRadix + d];
+          s_hist[w * kRadix + d] = run;
+          run += c;
+        }
+    }
+    __syncthreads();
+    for (int i0 = c0; i0 < c1; i0 += 32) {  // uniform over the warp
+      const int i = i0 + lane;
+      const bool valid = i < c1;
+      const unsigned long long v = valid ? a[i] : 0ull;
+      const unsigned dg = valid ? ((unsigned)(v >> shift) & 0xffu) : 0x100u;
+      const unsigned peers = __match_any_sync(0xffffffffu, dg);
+      const unsigned lower = peers & lt;
+      const unsigned at = valid ? h[dg] : 0u;
+      __syncwarp();
+      if (valid) {
+        b[at + __popc(lower)] = v;
+        if (lower == 0u) h[dg] = at + __popc(peers);
+      }
+      __syncwarp();
+    }
+    __syncthreads();
+    unsigned long long* t = a;
+    a = b;
+    b = t;
+  }
+  return a;
+}
+
+// load -> sort -> sorted ids back in place.  Inlined twice: with shared-memory buffers and with global scratch.
+// The composite is (key - kmin) << 32 | id.  Depth ties are rare, so the tile is first sorted on the KEY digits only
+// (about half the passes: ties come out in bucket order), then every run of equal keys is put in id order by the thread
+// that owns its first element (insertion sort, runs of up to kMaxRun).  A longer run (all-equal or quantised depths)
+// makes the CTA sort the whole composite instead, id digits included.
+constexpr int kMaxRun = 32;
+__device__ __forceinline__ void pair_sort_tile(unsigned long long* a, unsigned long long* b, int2 range,
+                                               unsigned kmin, const unsigned* __restrict__ tile_keys,
+                                               int* __restrict__ gids_sorted, unsigned* s_hist, int* s_warp,
+                                               unsigned long long* s_or_and) {
+  const int n = range.y - range.x;
+  unsigned long long o = 0ull, an = ~0ull;
+  for (int i0 = threadIdx.x; i0 < n; i0 += 4 * kPairThreads) {  // 4 independent load pairs in flight per thread
+    unsigned k[4];
+    int g[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int i = i0 + u * kPairThreads;
+      k[u] = (i < n) ? tile_keys[range.x + i] : kmin;
+      g[u] = (i < n) ? gids_sorted[range.x + i] : 0;
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int i = i0 + u * kPairThreads;
+      if (i < n) {
+        const unsigned long long c = ((unsigned long long)(k[u] - kmin) << 32) | (unsigned)g[u];
+        a[i] = c;
+        o |= c;
+        an &= c;
+      }
+    }
+  }
+  const unsigned olo = __reduce_or_sync(0xffffffffu, (unsigned)o), ohi = __reduce_or_sync(0xffffffffu, (unsigned)(o >> 32));
+  const unsigned alo = __reduce_and_sync(0xffffffffu, (unsigned)an),
+                 ahi = __reduce_and_sync(0xffffffffu, (unsigned)(an >> 32));
+  if ((threadIdx.x & 31) == 0) {
+    atomicOr(&s_or_and[0], ((unsigned long long)ohi << 32) | olo);
+    atomicAnd(&s_or_and[1], ((unsigned long long)ahi << 32) | alo);
+  }
+  __syncthreads();  // composites stored, OR / AND complete
+  const unsigned long long varying = s_or_and[0] & ~s_or_and[1];
+  unsigned long long* res = pair_radix_sort(a, b, n, varying & 0xffffffff00000000ull, s_hist, s_warp);
+  bool long_run = false;
+  for (int i = threadIdx.x; i < n; i += kPairThreads) {
+    const unsigned key = (unsigned)(res[i] >> 32);
+    if (i > 0 && (unsigned)(res[i - 1] >> 32) == key) continue;  // not the first element of its run
+    int e = i + 1;
+    while (e < n && e - i <= kMaxRun && (unsigned)(res[e] >> 32) == key) ++e;
+    if (e - i > kMaxRun) {
+      long_run = true;
+    } else {
+      for (int j = i + 1; j < e; ++j) {  // same key: order by id
+        const unsigned long long v = res[j];
+        int p = j - 1;
+        while (p >= i && res[p] > v) {
+          res[p + 1] = res[p];
+          --p;
+        }
+        res[p + 1] = v;
+      }
+    }
+  }
+  if (__syncthreads_or(long_run)) res = pair_radix_sort(res, res == a ? b : a, n, varying, s_hist, s_warp);
+  for (int i = threadIdx.x; i < n; i += kPairThreads) gids_sorted[range.x + i] = (int)(unsigned)res[i];
+}
+
+__global__ void __launch_bounds__(kPairThreads, 2) tile_pair_sort_kernel(
+    const int* __restrict__ order, const int2* __restrict__ tile_bins,
+    const unsigned* __restrict__ key_bits /* [5] = ~min visible key */, const unsigned* __restrict__ tile_keys,
+    int* __restrict__ gids_sorted, float* __restrict__ records /* scratch of oversized tiles */) {
+  extern __shared__ unsigned long long s_pairs[];  // [2][kPairCap] | [kPairWarps][kRadix] unsigned
+  __shared__ int s_warp[33];
+  __shared__ unsigned long long s_or_and[2];
+  const int tile = order ? order[blockIdx.x] : (int)blockIdx.x;
+  const int2 range = tile_bins[tile];
+  const int n = range.y - range.x;
+  if (n <= 1) return;  // uniform over the CTA; one pair is sorted
+  if (threadIdx.x == 0) {
+    s_or_and[0] = 0ull;
+    s_or_and[1] = ~0ull;
+  }
+  __syncthreads();
+  const unsigned kmin = ~key_bits[5];
+  unsigned* s_hist = reinterpret_cast<unsigned*>(s_pairs + 2 * kPairCap);
+  if (n <= kPairCap) {
+    pair_sort_tile(s_pairs, s_pairs + kPairCap, range, kmin, tile_keys, gids_sorted, s_hist, s_warp, s_or_and);
+  } else {
+    unsigned long long* a = reinterpret_cast<unsigned long long*>(records + 12 * (size_t)range.x);  // 48 B per slot
+    pair_sort_tile(a, a + n, range, kmin, tile_keys, gids_sorted, s_hist, s_warp, s_or_and);
+  }
+}
+
+// Late colours (gb_bin_tiles_pack_ev with an event): tile_scatter leaves the colour quarter of the per-Gaussian records
 // empty and this kernel fills it once the colours exist — colours are the only input of the binning that comes from
-// the shade, so everything before it can run beside the shade forward.
+// the shade, so everything before it can run beside the shade forward.  rank_of = NULL: the table is indexed by id.
 __global__ void __launch_bounds__(256) rec_colors_kernel(int G, const int* __restrict__ radii,
                                                          const int* __restrict__ rank_of,
                                                          const float* __restrict__ colors3,
                                                          const float* __restrict__ depths, float4* __restrict__ rec_by_rank) {
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= G || radii[g] <= 0) return;
-  rec_by_rank[3 * (size_t)rank_of[g] + 2] = make_float4(colors3[3 * (size_t)g], colors3[3 * (size_t)g + 1],
-                                                       colors3[3 * (size_t)g + 2], depths[g]);
+  const size_t at = rank_of ? (size_t)rank_of[g] : (size_t)g;
+  rec_by_rank[3 * at + 2] = make_float4(colors3[3 * (size_t)g], colors3[3 * (size_t)g + 1], colors3[3 * (size_t)g + 2],
+                                        depths[g]);
 }
 
+// rank_to_gid = NULL (per-tile sort path): `ranks_sorted` already holds the sorted Gaussian ids (it is gids_sorted),
+// the table is indexed by id and only the records are written.
 __global__ void __launch_bounds__(256) gather_records_kernel(long long cap, const int* __restrict__ n_dev,
-                                                             const int* __restrict__ ranks_sorted,
-                                                             const int* __restrict__ rank_to_gid,
-                                                             const float4* __restrict__ rec_by_rank,
-                                                             int* __restrict__ gids_sorted, float4* __restrict__ rec) {
+                                                             const int* ranks_sorted, const int* __restrict__ rank_to_gid,
+                                                             const float4* __restrict__ rec_by_rank, int* gids_sorted,
+                                                             float4* __restrict__ rec) {
   const long long n = min((long long)*n_dev, cap);
   const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // float4 index: record j / 3, part j % 3
   if (j >= 3 * n) return;
@@ -837,7 +1029,7 @@ __global__ void __launch_bounds__(256) gather_records_kernel(long long cap, cons
   const int part = (int)(j - 3 * i);
   const int r = ranks_sorted[i];
   rec[j] = gb::ld_nc_f4(rec_by_rank + 3 * (size_t)r + part);
-  if (part == 0) gids_sorted[i] = rank_to_gid[r];
+  if (rank_to_gid && part == 0) gids_sorted[i] = rank_to_gid[r];
 }
 
 struct Layout {
@@ -880,6 +1072,14 @@ int tile_sort_mode() {
   }
   return g_tile_sort_mode;
 }
+int g_bin_sort_mode = -1;  // 0: per-tile (depth key, id) sort (default), 1: depth ranks + per-tile rank ordering
+int bin_sort_mode() {
+  if (g_bin_sort_mode < 0) {
+    const char* e = getenv("GOLIATH_B200_BINSORT");
+    g_bin_sort_mode = (e && strcmp(e, "rank") == 0) ? 1 : 0;
+  }
+  return g_bin_sort_mode;
+}
 int g_rank_sort_mode = -1;  // 0: cooperative LSD sort, 1: four separate radix passes (round 1), 2: bucket ranking (+ fallback)
 int rank_sort_mode() {
   if (g_rank_sort_mode < 0) {
@@ -905,7 +1105,7 @@ int launch_rank_sort(int G, int ctas, const float* xys, const float* depths, con
                      int block_width, int smem_tiles, unsigned* keys_a, unsigned* keys_b, int* vals_a, int* vals_b,
                      unsigned* hist, int* counts, int* buckets, unsigned* sync, int* rank_to_gid, int* rank_of, cudaStream_t s) {
   const size_t hs = (size_t)ctas * kRadix;
-  depth_keys_kernel<kRankBlock * kItems><<<ctas, kGaussBlock, (size_t)smem_tiles * 4, s>>>(
+  depth_keys_kernel<kRankBlock * kItems, true><<<ctas, kGaussBlock, (size_t)smem_tiles * 4, s>>>(
       G, (const float2*)xys, depths, radii, tbx, tby, block_width, smem_tiles, keys_a, hist, counts, sync);
   const int mode = rank_sort_mode();
   if (mode == 2) {  // bucket ranking
@@ -958,8 +1158,14 @@ int opt_in_smem(K kernel, bool* done) {
 
 }  // namespace
 
-// Depth-rank sort of gb_bin_tiles_pack: 0 = one cooperative kernel over the varying key bits (default), 1 = four
-// radix passes as separate launches (round 1).  Identical outputs; the switch exists for A/B timing and the tests.
+// Ordering of gb_bin_tiles_pack[_ev]: 0 = per-tile sort of (depth key, id) pairs (default), 1 = depth ranks + per-tile
+// rank ordering, whose variants the rank / tile sort modes below select (gb_bin_tiles_ranked always uses ranks).
+// Identical outputs; the switches exist for A/B timing and the tests.
+GB_API int gb_get_bin_sort_mode(void) { return bin_sort_mode(); }
+GB_API void gb_set_bin_sort_mode(int mode) { g_bin_sort_mode = mode ? 1 : 0; }
+// Depth-rank sort of the rank path: 0 = one cooperative kernel over the varying key bits (default), 1 = four
+// radix passes as separate launches (round 1), 2 = bucket ranking.  Per-tile rank ordering: 0 = bitmap sort + grid-wide
+// record gather (default), 1 = one kernel per tile (round 1).
 GB_API int gb_get_tile_sort_mode(void) { return tile_sort_mode(); }
 GB_API void gb_set_tile_sort_mode(int mode) { g_tile_sort_mode = mode ? 1 : 0; }
 GB_API int gb_get_rank_sort_mode(void) { return rank_sort_mode(); }
@@ -1051,22 +1257,37 @@ static int bin_tiles_impl(int G, const float* xys, const float* depths, const in
   const int items = rank_items(G);
   const int ctas = gb::cdiv(G, kRankBlock * items);
   const int smem_tiles = (T <= kMaxSmemTiles) ? T : 0;
+  // per-tile sort of (depth key, id) pairs: no depth ranks; the by-rank table becomes a by-id table
+  const bool by_id = !ranked && bin_sort_mode() == 0;
   static bool s_opt_k8[64] = {}, s_opt_k16[64] = {}, s_opt_scat[64] = {}, s_opt_sort[64] = {}, s_opt_sort2[64] = {};
+  static bool s_opt_k8i[64] = {}, s_opt_k16i[64] = {}, s_opt_scati[64] = {}, s_opt_pair[64] = {};
   if ((size_t)smem_tiles * 8 > 40 * 1024) {
-    int e = (items == 8) ? opt_in_smem(depth_keys_kernel<kRankBlock * 8>, s_opt_k8)
-                         : opt_in_smem(depth_keys_kernel<kRankBlock * 16>, s_opt_k16);
+    int e = by_id ? ((items == 8) ? opt_in_smem(depth_keys_kernel<kRankBlock * 8, false>, s_opt_k8i)
+                                  : opt_in_smem(depth_keys_kernel<kRankBlock * 16, false>, s_opt_k16i))
+                  : ((items == 8) ? opt_in_smem(depth_keys_kernel<kRankBlock * 8, true>, s_opt_k8)
+                                  : opt_in_smem(depth_keys_kernel<kRankBlock * 16, true>, s_opt_k16));
     if (e) return e;
-    e = opt_in_smem(tile_scatter_kernel, s_opt_scat);
+    e = by_id ? opt_in_smem(tile_scatter_kernel<true>, s_opt_scati) : opt_in_smem(tile_scatter_kernel<false>, s_opt_scat);
     if (e) return e;
   }
 
   GB_CUDA(cudaMemsetAsync(ws, 0, l.zero_bytes, s));
-  const int es = (items == 8)
-                     ? launch_rank_sort<8>(G, ctas, xys, depths, radii, tbx, tby, block_width, smem_tiles, keys_a, keys_b,
-                                           vals_a, vals_b, hist, counts, (int*)(ws + l.buckets), sync, rank_to_gid, rank_of, s)
-                     : launch_rank_sort<16>(G, ctas, xys, depths, radii, tbx, tby, block_width, smem_tiles, keys_a, keys_b,
-                                            vals_a, vals_b, hist, counts, (int*)(ws + l.buckets), sync, rank_to_gid, rank_of, s);
-  if (es) return es;
+  if (by_id) {
+    if (items == 8)
+      depth_keys_kernel<kRankBlock * 8, false><<<ctas, kGaussBlock, (size_t)smem_tiles * 4, s>>>(
+          G, (const float2*)xys, depths, radii, tbx, tby, block_width, smem_tiles, nullptr, nullptr, counts, sync);
+    else
+      depth_keys_kernel<kRankBlock * 16, false><<<ctas, kGaussBlock, (size_t)smem_tiles * 4, s>>>(
+          G, (const float2*)xys, depths, radii, tbx, tby, block_width, smem_tiles, nullptr, nullptr, counts, sync);
+    gb::count_launches(1);
+  } else {
+    const int es = (items == 8)
+                       ? launch_rank_sort<8>(G, ctas, xys, depths, radii, tbx, tby, block_width, smem_tiles, keys_a, keys_b,
+                                             vals_a, vals_b, hist, counts, (int*)(ws + l.buckets), sync, rank_to_gid, rank_of, s)
+                       : launch_rank_sort<16>(G, ctas, xys, depths, radii, tbx, tby, block_width, smem_tiles, keys_a, keys_b,
+                                              vals_a, vals_b, hist, counts, (int*)(ws + l.buckets), sync, rank_to_gid, rank_of, s);
+    if (es) return es;
+  }
   int* n_total = n_out ? n_out : (int*)(sync + 3);  // the record gather below needs the count on the device
   tile_scan_kernel<<<1, 1024, 0, s>>>(T, (long long)cap, counts, (int2*)tile_bins, cursor, n_total, overflow);
   gb::count_launches(1);
@@ -1074,12 +1295,36 @@ static int bin_tiles_impl(int G, const float* xys, const float* depths, const in
   const int e = tile_sched ? gb_tile_schedule(T, tile_bins, tile_order, stream)
                            : gb_tile_order(T, tile_bins, tile_order, stream);
   if (e) return e;
-  const bool split = ranked || tile_sort_mode() == 0;
-  const bool late = split && colors_ready;  // the colour quarter of the by-rank records is filled after the tile sort
+  const bool split = by_id || ranked || tile_sort_mode() == 0;
+  const bool late = split && colors_ready;  // the colour quarter of the per-Gaussian records is filled after the tile sort
   if (!late && colors_ready) GB_CUDA(cudaStreamWaitEvent(s, (cudaEvent_t)colors_ready, 0));
-  tile_scatter_kernel<<<gb::cdiv(G, kGaussBlock * kScatItems), kGaussBlock, (size_t)smem_tiles * 8, s>>>(
+  const int scat_ctas = gb::cdiv(G, kGaussBlock * kScatItems);
+  if (by_id) {
+    // tile_ranks receives the depth keys, gids_sorted the ids; the table at rec_by_rank is indexed by id
+    tile_scatter_kernel<true><<<scat_ctas, kGaussBlock, (size_t)smem_tiles * 8, s>>>(
+        G, (const float2*)xys, radii, nullptr, conics, late ? nullptr : colors3, depths, opacity, compensation, tbx, tby,
+        block_width, (long long)cap, smem_tiles, cursor, tile_ranks, gids_sorted, rec_by_rank);
+    if (cap > 0) {
+      const int e2 = opt_in_smem(tile_pair_sort_kernel, s_opt_pair);
+      if (e2) return e2;
+      tile_pair_sort_kernel<<<T, kPairThreads, kPairSmem, s>>>(tile_order, (const int2*)tile_bins, sync,
+                                                               (const unsigned*)tile_ranks, gids_sorted, records);
+    }
+    if (late) {
+      GB_CUDA(cudaStreamWaitEvent(s, (cudaEvent_t)colors_ready, 0));
+      rec_colors_kernel<<<gb::cdiv(G, 256), 256, 0, s>>>(G, radii, nullptr, colors3, depths, rec_by_rank);
+      gb::count_launches(1);
+    }
+    if (cap > 0)
+      gather_records_kernel<<<(unsigned)gb::cdiv64(3 * cap, 256), 256, 0, s>>>((long long)cap, n_total, gids_sorted, nullptr,
+                                                                               rec_by_rank, gids_sorted, (float4*)records);
+    gb::count_launches(3);
+    GB_CHECK_LAUNCH();
+    return 0;
+  }
+  tile_scatter_kernel<false><<<scat_ctas, kGaussBlock, (size_t)smem_tiles * 8, s>>>(
       G, (const float2*)xys, radii, rank_of, conics, late ? nullptr : colors3, depths, opacity, compensation, tbx, tby,
-      block_width, (long long)cap, smem_tiles, cursor, tile_ranks, rec_by_rank);
+      block_width, (long long)cap, smem_tiles, cursor, tile_ranks, nullptr, rec_by_rank);
   const int words = gb::cdiv(G, 32);
   const int chunk = gb::cdiv(words, kSortThreads) | 1;
   const size_t smem = (size_t)words * 4;

@@ -90,8 +90,8 @@ class _RenderFused(Function):
                 order = torch.empty(L.gb_tile_schedule_ints(T) if sched else T, **i32)
                 records = torch.empty(cap, 12, **f32)
                 if BINNING == "buckets" and L.gb_bin_tiles_supported(G):
-                    # depth ranks + per-tile buckets ordered by a rank bitmap (csrc/splat_bin_tiles.cu): same bins,
-                    # ids and records as the key sort below, without sorting the intersection keys
+                    # per-tile buckets, each sorted on chip by (depth key, id) (csrc/splat_bin_tiles.cu): same bins,
+                    # ids and records as the key sort below, without a global sort of the intersection keys
                     bins = torch.empty(T, 2, **i32)
                     ws = _workspace(dev, L.gb_bin_tiles_workspace_bytes(G, T, cap))
                     _lib.check(L.gb_bin_tiles_pack(G, _lib.ptr(xys), _lib.ptr(depths), _lib.ptr(radii),

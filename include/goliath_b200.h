@@ -162,12 +162,18 @@ int gb_pack_records_fused_dn(int64_t cap, const int32_t* n_dev, const int32_t* g
                              const float* conics, const float* colors3, const float* depths, const float* opacity,
                              const float* compensation, float* records, void* stream);
 
-/* depth ranks inside gb_bin_tiles_pack: 0 = one cooperative LSD kernel over the key bits that vary (default), 1 = four
+/* ordering inside gb_bin_tiles_pack / gb_bin_tiles_pack_ev: 0 = each tile's (depth key, id) pairs sorted in shared memory
+ * by one CTA, no depth ranks (default); 1 = depth ranks of all Gaussians + per-tile rank ordering, the path the rank and
+ * tile sort modes below select between (gb_bin_tiles_ranked always takes it).  Identical outputs.
+ * GOLIATH_B200_BINSORT=tile|rank. */
+int gb_get_bin_sort_mode(void);
+void gb_set_bin_sort_mode(int mode);
+/* depth ranks of the rank path: 0 = one cooperative LSD kernel over the key bits that vary (default), 1 = four
  * radix passes as separate launches (round 1), 2 = 2048 key buckets + in-bucket ranking of the visible Gaussians (a
  * device flag hands degenerate depth distributions to the cooperative sort; measured slower).  Identical outputs.
  * GOLIATH_B200_RANKSORT=coop|passes|buckets. */
 int gb_get_rank_sort_mode(void);
-/* per-tile ordering inside gb_bin_tiles_pack: 0 = bitmap sort per tile + one grid-wide record gather (default), 1 = one
+/* per-tile rank ordering of the rank path: 0 = bitmap sort per tile + one grid-wide record gather (default), 1 = one
  * kernel per tile doing both (round 1).  Identical outputs.  GOLIATH_B200_TILESORT=split|fused. */
 int gb_get_tile_sort_mode(void);
 void gb_set_tile_sort_mode(int mode);
@@ -176,8 +182,9 @@ void gb_set_rank_sort_mode(int mode);
 /* Bucket binning of the fused render (csrc/splat_bin_tiles.cu): replaces, for the fused path, the whole of gsplat
  * 0.1.11 bin_and_sort_gaussians (compute_cumulative_intersects, map_gaussian_to_intersects, torch.sort,
  * get_tile_bin_edges — call sites ca_code/utils/render_gsplat.py:65-78,90-104) plus the record packing, with the same
- * bit-exact outputs: Gaussians are depth-ranked once (G keys), intersections are bucketed per tile with atomics, and
- * each tile's bucket is ordered with a rank bitmap in shared memory.  Outputs: tile_bins [T,2], tile_order [T]
+ * bit-exact outputs: intersections are bucketed per tile with atomics as (depth key, id) pairs, and each tile's bucket
+ * is sorted by one CTA in shared memory (a tile too long for it sorts in its own slots of `records`, which the final
+ * record gather overwrites).  Outputs: tile_bins [T,2], tile_order [T]
  * (tile_sched = 1: an SM-affine schedule of gb_tile_schedule_ints(T) int32 instead, see gb_tile_schedule),
  * gids_sorted [cap], records [cap,12]; n_out (device int32, may be NULL) = true intersection count; *overflow = 1
  * when it exceeds cap (the excess is dropped).  Sync-free, never allocates, capturable in a CUDA graph. */
